@@ -14,6 +14,10 @@ GPU -> 10240 erasure blocks; inputs are far larger than the 126 MB L2, so no exp
   configs   BASELINE configs 3, 4 and 5 (device-resident kernels + config 4 through mec_heal_batch), each with its own
             roofline fraction and a check against the encode outputs
   cpu_baseline / --impl reference   the C oracle's SIMD path on a persistent, pinned pthread pool over all host cores
+
+  --dump-outputs DIR   after the timed steps, rank 0 writes a fixed sample of what the last timed step returned (parity shards
+            and digests in float32, the sampled block indices in float64) as DIR/<name>.npy; the input stream is seeded, so two
+            builds can be compared array for array
 """
 import argparse
 import ctypes as C
@@ -40,6 +44,9 @@ METRIC = "fused RS(12,4) encode + HighwayHash256 bitrot, 1 MiB blocks"
 # SASS of fused_rs_hh_kernel<GfStatic<12,4>,1,6,4,0,1>; profiles/r2_sass_loop.md says how to recount): 172 GF + 224 HighwayHash + 9 loop
 ALU_WARP_INSTR_PER_TILE_BLOCK = 405
 CPU_BLOCKS = int(os.environ.get("MEC_CPU_BLOCKS", "4096"))   # CPU arm: 4 GiB source per pass — larger than any last-level cache
+# --dump-outputs sample, as float32: parity of 16 blocks (22.4 MB) and digests of up to 12288 blocks (25.2 MB; all of the default
+# 10240), so the files stay under 64 MB whatever --blocks is
+DUMP_PARITY_BLOCKS, DUMP_DIGEST_BLOCKS, DUMP_SEED = 16, 12288, 0x4D494E494F03
 
 
 def workload_config(nblocks, world):
@@ -107,8 +114,7 @@ class CpuArm:
 
     def __init__(self, threads, nblocks=CPU_BLOCKS):
         import oracle_lib as o
-        o.build()
-        self.L = o.lib()
+        self.L = o.lib()   # built by build(): the benchmark compiles nothing into the tree
         self.threads, self.nblocks = threads, nblocks
         self.pool = self.L.orc_pool_new(threads)
         # untouched anonymous memory: np.empty does not touch the pages, the workers do (first touch = node-local)
@@ -158,6 +164,21 @@ def ptr_array(arrs):
     return (C.c_void_p * len(arrs))(*[(a.ctypes.data if a is not None else None) for a in arrs])
 
 
+def dump_outputs(out_dir, par, dig, nblocks):
+    """What a caller of the timed encode receives, for a seeded sample of blocks: parity.npy [block, parity shard, S] (without the
+    row pitch padding, which the kernel does not write), digests.npy [block, shard, 32], and the sampled block indices."""
+    import torch
+    rng = np.random.default_rng(DUMP_SEED)
+    pb, db = (np.arange(nblocks) if n >= nblocks else np.sort(rng.choice(nblocks, n, replace=False))
+              for n in (DUMP_PARITY_BLOCKS, DUMP_DIGEST_BLOCKS))
+    out = {"parity": par.view(nblocks, M, -1)[torch.from_numpy(pb).to(par.device), :, :S].float().cpu().numpy(),
+           "digests": dig[torch.from_numpy(db).to(dig.device)].float().cpu().numpy(),
+           "parity_blocks": pb.astype(np.float64), "digest_blocks": db.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -170,6 +191,7 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -246,6 +268,8 @@ def main():
     kern_ms = [a.elapsed_time(b) for a, b in evs]
     ms_per_step = total_ms / args.steps
     value = world * nbytes / GiB / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, par, dig, nblocks)
 
     # ---- input scatter over NVLink (SURVEY §8e): rank 0 owns a single-source stream and hands every rank its slice
     # with NCCL; timed separately from the kernel metric (the data path itself has no collective)
@@ -273,7 +297,6 @@ def main():
     oracle_leg = rank == 0 and not args.no_cpu
     if oracle_leg:
         import oracle_lib as o
-        o.build()
         verified = True
         for b in (0, nblocks // 2, nblocks - 1):
             blk = src[b * BS:(b + 1) * BS].cpu().numpy()
